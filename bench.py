@@ -185,6 +185,29 @@ def cpu_strong_forward(params, x, segments, steps=3, warmup=1, threads=None):
     return steps / dt, dt / steps * 1e3, threads, fc8
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+PARAM_SAMPLE = 1 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the arrays the timed path returned in its last step, one DIR/<name>.npy each, so that two
+    builds run with the same arguments (hence the same seeded inputs and weights) can be compared output for output"""
+    arrays = {k: np.ascontiguousarray(v, np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
+def param_sample(net):
+    """a fixed, seeded sample of PARAM_SAMPLE elements of all parameter blobs (layer order, flattened)"""
+    flat = np.concatenate([np.asarray(b.data, np.float32).ravel() for blobs in net.params.values() for b in blobs])
+    idx = np.sort(np.random.default_rng(0).choice(flat.size, size=min(PARAM_SAMPLE, flat.size), replace=False))
+    return flat[idx]
+
+
 TRAIN_SOLVER = """base_lr: 0.001 lr_policy: "step" gamma: 0.1 stepsize: 24000 max_iter: 60000 iter_size: 1
 momentum: 0.9 weight_decay: 0.0005 clip_gradients: 40 solver_type: NESTEROV"""   # models_ECO_Lite/kinetics/solver.prototxt (iter_size 1)
 
@@ -268,6 +291,11 @@ def train_main(a, rank, local_rank, world):
     ms_total = grp.max_over_ranks(e0.elapsed_time(e1))
     ms_step = ms_total / a.steps
     value = world * batch * a.steps / (ms_total / 1e3)
+    if a.dump_outputs and rank == 0:
+        # the last timed step's loss and logits, and the parameters its update left behind
+        dump_outputs(a.dump_outputs, {"loss": np.array([losses[-1]], np.float64),
+                                      "fc8": np.array(net.blobs["fc8"].data, np.float32),
+                                      "params_sample": param_sample(net)})
     # e2e: the batch comes from the input blob's pinned host mirror every step (what a data layer would fill), loss read back
     host_in = net.blobs["data"].data
     host_in[...] = frames.cpu().numpy()
@@ -347,7 +375,12 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-calibrate", action="store_true", help="skip the BN calibration forwards of the weight harness (ncu captures)")
     ap.add_argument("--h2d-chunks", type=int, default=0, help="blocking forward: 0 auto (4 sub-batches), 1 unsplit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy: "
+                         "infer: fc8 logits; train: loss, fc8 logits and a seeded sample of the updated parameters")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs records the GPU arm's outputs; the reference arm has none to record")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -441,6 +474,8 @@ def main():
     # logits of clip 0 from this plan (graph replay, production options), checked against the oracle further down
     dev_logits0 = np.array(net.blobs["fc8"].data[0:1], np.float32, copy=True)
     clip0 = frames[:N].cpu().numpy()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"fc8": net.blobs["fc8"].data})
 
     # ---------------- e2e: host buffers in, logits out, copies inside the timed region ----------------
     host_in = net.blobs["data"].data  # pinned host mirror of the input blob (what caffe's data layer fills)

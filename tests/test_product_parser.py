@@ -1,37 +1,38 @@
 """Every net definition the reference ships loads through the PRODUCT's own prototxt parser and graph
 builder (csrc/prototxt.hpp, Net::build_graph -- no GPU needed for construction), and the caffe-visible
 layer / blob names -- including the automatically inserted Split layers (insert_splits.cpp:13-142) --
-agree with the oracle's independent restatement of InsertSplits.  Runs wherever /root/reference is mounted."""
-import glob
-import os
-
+agree with the oracle's independent restatement of InsertSplits.  The nets are rebuilt from
+tests/golden/reference_nets.json; each rebuild must parse to the reference file's tree (SHA-256)."""
 import pytest
 
-from oracle import refnet
+from oracle import prototxt, refnet
+from eco_testlib import reference_net_text, reference_nets, tree_sha256
 
-REF = "/root/reference"
-FILES = sorted(glob.glob(os.path.join(REF, "models_ECO_*", "*", "*.prototxt")))
-NETS = [f for f in FILES if os.path.basename(f) != "solver.prototxt"]
+NETS = reference_nets()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
 def test_reference_tree_has_the_expected_nets():
-    names = {os.path.relpath(f, REF) for f in NETS}
+    names = {e["path"] for e in NETS}
     assert "models_ECO_Lite/ucf101/deploy.prototxt" in names
     assert "models_ECO_Full/kinetics/ECO_full.prototxt" in names or any("ECO_full" in n or "ECO_Full" in n for n in names)
     assert len(NETS) >= 9
+    for e in NETS:
+        assert tree_sha256(prototxt.parse(reference_net_text(e))) == e["sha256"], e["path"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
-@pytest.mark.parametrize("path", NETS, ids=[os.path.relpath(f, REF) for f in NETS])
+@pytest.mark.parametrize("entry", NETS, ids=[e["path"] for e in NETS])
 @pytest.mark.parametrize("phase", ["TEST", "TRAIN"])
-def test_product_parser_loads_reference_net(path, phase):
+def test_product_parser_loads_reference_net(entry, phase, tmp_path):
     import caffe
-    is_deploy = os.path.basename(path) == "deploy.prototxt"
+    is_deploy = not entry["data_layers"]   # declares its inputs instead of reading them through VideoData layers
     if is_deploy and phase == "TRAIN":
         pytest.skip("deploy nets are TEST-phase definitions")
-    net = caffe.Net(path, caffe.TEST if phase == "TEST" else caffe.TRAIN)
-    ref = refnet.RefNet(open(path).read(), phase=phase)
+    text = reference_net_text(entry)
+    assert tree_sha256(prototxt.parse(text)) == entry["sha256"]
+    path = tmp_path / "net.prototxt"
+    path.write_text(text)
+    net = caffe.Net(str(path), caffe.TEST if phase == "TEST" else caffe.TRAIN)
+    ref = refnet.RefNet(text, phase=phase)
     want_layers, want_blobs = ref.split_names()
     got_layers = list(net._layer_names)
     got_blobs = list(net._blob_names)

@@ -1,22 +1,14 @@
 """tools/gen_eco_prototxt.py must emit nets structurally identical to the reference's
-hand-written prototxts (checked whenever /root/reference is mounted), and the oracle's
-InsertSplits naming must follow caffe_3d/src/caffe/util/insert_splits.cpp."""
-import os
-
+hand-written prototxts (pinned by the SHA-256 of each file's parsed tree in
+tests/golden/reference_nets.json), and the oracle's InsertSplits naming must follow
+caffe_3d/src/caffe/util/insert_splits.cpp."""
 import pytest
 
 from oracle import prototxt, refnet
 import gen_eco_prototxt as gen
+from eco_testlib import norm_tree as norm, reference_net_text, reference_nets, tree_sha256
 
-REF = "/root/reference"
-
-
-def norm(v):
-    if isinstance(v, prototxt.Msg):
-        return {k: [norm(x) for x in vv] for k, vv in v.items()}
-    if isinstance(v, (int, float)) and not isinstance(v, bool):
-        return float(v)
-    return v
+REF_NETS = {e["path"]: e for e in reference_nets()}
 
 
 CASES = [
@@ -28,18 +20,13 @@ CASES = [
 ]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
 @pytest.mark.parametrize("path,make", CASES, ids=[c[0] for c in CASES])
 def test_generated_equals_reference(path, make):
-    ref = norm(prototxt.parse_file(os.path.join(REF, path)))
-    mine = norm(prototxt.parse(make()))
-    if ref.get("name") != mine.get("name"):
-        mine["name"] = ref["name"]  # net name differs per dataset; not part of the graph
-    assert ref.keys() == mine.keys()
-    assert len(ref["layer"]) == len(mine["layer"])
-    for a, b in zip(ref["layer"], mine["layer"]):
-        assert a == b, (a.get("name"), b.get("name"))
-    assert {k: v for k, v in ref.items() if k != "layer"} == {k: v for k, v in mine.items() if k != "layer"}
+    ref = REF_NETS[path]
+    mine = prototxt.parse(make())
+    mine["name"] = [ref["kwargs"]["net_name"]]  # net name differs per dataset; not part of the graph
+    assert len(mine["layer"]) == ref["layers"]
+    assert tree_sha256(mine) == ref["sha256"]
 
 
 def test_split_names_lite():
@@ -72,13 +59,16 @@ TRAIN_CASES = [
 ]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
 @pytest.mark.parametrize("path,make", TRAIN_CASES, ids=[c[0] for c in TRAIN_CASES])
 def test_generated_train_net_equals_reference_after_the_data_layers(path, make):
     """the train/test definition: everything behind the VideoData layers (which the generator replaces by the two net
     inputs they produce) must be the reference's graph: names, types, bottoms/tops, phase rules, every numeric parameter"""
-    ref = norm(prototxt.parse_file(os.path.join(REF, path)))
-    mine = norm(prototxt.parse(make()))
+    entry = REF_NETS[path]
+    text = make()
+    ref_tree = prototxt.parse(reference_net_text(entry, text))
+    assert tree_sha256(ref_tree) == entry["sha256"], "the generator no longer rebuilds " + path
+    ref = norm(ref_tree)
+    mine = norm(prototxt.parse(text))
     ref_layers = [l for l in ref["layer"] if l["type"] != ["VideoData"]]
     assert len(ref_layers) == len(mine["layer"])
     for a, b in zip(ref_layers, mine["layer"]):
